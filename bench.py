@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """bench.py -- warp + multiband-blend throughput of the B200 compositing path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2] [--dump-outputs DIR]
+
+`--dump-outputs DIR` (--impl ours, one GPU or --replicas) writes what the last timed step computed, see dump_outputs().
 
 One "step" = one pass of the hot path over one batch of synthetic frames for a fixed rig: fused warp of
 every image (+ validity mask), Gaussian/weight pyramids, per-band weighted accumulate + normalise + collapse,
@@ -301,6 +303,26 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 60_000_000  # the .npy files of --dump-outputs stay below 64 MB
+
+
+def dump_outputs(d, pano, mask):
+    """--dump-outputs: the panorama and mask of the last timed step, as float32 DIR/pano.npy (h x w x 3) and DIR/mask.npy
+    (h x w).  When they would exceed DUMP_BYTES, a fixed sample of pixels (the same for the same panorama size) stands for them:
+    DIR/pano_sample.npy (k x 3), DIR/mask_sample.npy (k) and their flat pixel indices DIR/pixel_index.npy (float64)."""
+    os.makedirs(d, exist_ok=True)
+    h, w = mask.shape
+    per_pixel = 4 * 4  # float32 r, g, b, mask
+    if h * w * per_pixel <= DUMP_BYTES:
+        np.save(os.path.join(d, "pano.npy"), pano.astype(np.float32))
+        np.save(os.path.join(d, "mask.npy"), mask.astype(np.float32))
+        return
+    idx = np.sort(np.random.default_rng(0).choice(h * w, DUMP_BYTES // (per_pixel + 8), replace=False))
+    np.save(os.path.join(d, "pano_sample.npy"), pano.reshape(-1, 3)[idx].astype(np.float32))
+    np.save(os.path.join(d, "mask_sample.npy"), mask.reshape(-1)[idx].astype(np.float32))
+    np.save(os.path.join(d, "pixel_index.npy"), idx.astype(np.float64))
+
+
 def set_extras(comp):
     """--extras: the other two FINAL-resolution steps of the pipeline fused into the step (SURVEY 8f f1, f2): a
     synthetic exposure gain map (one sample per 32x32 block, as gain_blocks estimates) and a LOW-resolution seam mask
@@ -400,6 +422,8 @@ def run_ours(args, rank, local_rank, world):
     for c2 in extra:
         c2.sync()
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:  # the steps were dealt round-robin: the last one ran on this compositor
+        dump_outputs(args.dump_outputs, *([comp] + extra)[(args.steps - 1) % (1 + len(extra))].download())
     dist.barrier()
     worst_ms = dist.max(total_ms)
     total_mpix = dist.sum(mpix_rank)
@@ -715,11 +739,15 @@ def main():
     ap.add_argument("--replicas", action="store_true", help="N > 1: one independent panorama per GPU instead of one sharded panorama")
     ap.add_argument("--extras", action="store_true", help="also fuse exposure gains and seam masks into the step (SURVEY 8f f1, f2)")
     ap.add_argument("--scale-down", type=int, default=1, help="debug: shrink the workload (not a valid measurement)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the panorama and mask of the last timed step (rank 0) as .npy files to DIR; "
+                                                          "--impl ours on one GPU or with --replicas only (not the sharded or reference paths)")
     args = ap.parse_args()
     global SCALE_DOWN
     SCALE_DOWN = args.scale_down
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank, local_rank, world = dist_env()
+    if args.dump_outputs and (args.impl == "reference" or (world > 1 and not args.replicas)):
+        ap.error("--dump-outputs: only the single-panorama path (--impl ours on one GPU, or --replicas)")
     if args.impl == "reference":
         run_reference(args, rank, world)
     elif world > 1 and not args.replicas:

@@ -34,11 +34,23 @@ def emu_lib():
 
 @pytest.fixture()
 def use_emu(emu_lib, monkeypatch):
-    """Route the Python drop-ins through the emulation library for this test only."""
-    from stitching_b200 import _lib
+    """Route the Python drop-ins through the emulation library for this test only.
 
+    Pooled page-locked buffers (host_pool) and device twins (device_array) are released through whichever library is bound
+    at that moment, so the ones left over are released on each side of the switch, each by the library that made them:
+    the emulation's cudaFree is free(), the real one's is not."""
+    import gc
+
+    from stitching_b200 import _lib, host_pool
+
+    def release_leftovers():
+        gc.collect()
+        host_pool.trim()
+
+    release_leftovers()
     monkeypatch.setattr(_lib, "_lib", emu_lib)
-    return emu_lib
+    yield emu_lib
+    release_leftovers()
 
 
 @pytest.fixture(scope="session")

@@ -18,12 +18,14 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
+sys.path.insert(0, os.path.join(HERE, ".."))
 sys.path.insert(0, "/root/reference")
 
 import cv2 as cv  # noqa: E402
 from stitching.blender import Blender as RefBlender  # noqa: E402
 from stitching.warper import Warper as RefWarper  # noqa: E402
 
+import replay  # noqa: E402
 from stitching_b200 import rigs  # noqa: E402
 
 
@@ -68,6 +70,7 @@ def gen_warp():
                        [s * np.sin(th), s * np.cos(th), [-7.75, 40.0, -33.5][k]], [0, 0, 1]], np.float32)
         cases.append(("affine", rigs.Camera(1.0, 1.0, 0.0, 0.0, Hm), 1.0, [1.0, 1.0, 0.75][k]))
     out = {"n": len(cases)}
+    src_sha = hashlib.sha256()  # the sources are drawn again from the seed (replay.warp_cases), not stored
     for i, (wtype, cam, scale, aspect) in enumerate(cases):
         img = rng.integers(0, 256, (H, W, 3), dtype=np.uint8)
         wr = RefWarper(wtype)
@@ -77,10 +80,11 @@ def gen_warp():
         out[f"R_{i}"] = cam.R
         out[f"scale_{i}"] = np.float64(scale)
         out[f"aspect_{i}"] = np.float64(aspect)
-        out[f"src_{i}"] = img
+        src_sha.update(img.tobytes())
         out[f"roi_{i}"] = np.array(wr.warp_roi((W, H), cam, aspect), np.int64)
-        out[f"img_{i}"] = wr.warp_image(img, cam, aspect)
-        out[f"mask_{i}"] = wr.create_and_warp_mask((W, H), cam, aspect)
+        replay.pack(out, f"img_{i}", wr.warp_image(img, cam, aspect))
+        replay.pack(out, f"mask_{i}", wr.create_and_warp_mask((W, H), cam, aspect))
+    out["src_sha256"] = src_sha.hexdigest()
     np.savez_compressed(os.path.join(HERE, "golden_warp.npz"), **out)
     print("warp cases", len(cases))
 
@@ -196,8 +200,8 @@ def gen_e2e():
         out[f"{name}_input_sha256"] = h.hexdigest()
         out[f"{name}_corners"] = np.array(corners, np.int64)
         out[f"{name}_sizes"] = np.array(sizes, np.int64)
-        out[f"{name}_pano"] = pano
-        out[f"{name}_pmask"] = pmask
+        replay.pack(out, f"{name}_pano", pano)
+        replay.pack(out, f"{name}_pmask", pmask)
         print(name, "pano", pano.shape)
     np.savez_compressed(os.path.join(HERE, "golden_e2e.npz"), **out)
 

@@ -29,15 +29,58 @@ def assert_exact(got, exp, what):
     assert n == 0, msg
 
 
+PACK_WHOLE_BYTES = 2048  # larger arrays are stored as shape + sha256 + a sample, so that a golden file stays small
+PACK_SAMPLE = 64
+
+
+def _sample_index(size):
+    return np.sort(np.random.default_rng(size).choice(size, min(size, PACK_SAMPLE), replace=False))
+
+
+def pack(out, key, arr):
+    """Store the expected array `arr` under `key` in the dict `out` (later np.savez_compressed): whole when small, else one
+    string "dtype shape sha256 sample" -- the sha256 of all its values and, in hex, a fixed sample of them (for the report
+    when they differ)."""
+    arr = np.ascontiguousarray(arr)
+    if arr.nbytes <= PACK_WHOLE_BYTES:
+        out[key] = arr
+        return
+    sample = arr.reshape(-1)[_sample_index(arr.size)]
+    out[f"{key}__digest"] = np.bytes_(" ".join([str(arr.dtype), "x".join(str(d) for d in arr.shape), hashlib.sha256(arr.tobytes()).hexdigest(),
+                                                sample.tobytes().hex()]))
+
+
+def assert_golden(got, g, key, what):
+    """`got` equals, value for value, the array pack() stored under `key` in the loaded golden file `g`."""
+    if key in g.files:
+        assert_exact(got, g[key], what)
+        return
+    dtype, shape, sha, sample = g[f"{key}__digest"].item().decode().split(" ")
+    got = np.ascontiguousarray(got)
+    shape = tuple(int(d) for d in shape.split("x"))
+    assert got.shape == shape, f"{what}: shape {got.shape} != {shape}"
+    assert str(got.dtype) == dtype, f"{what}: dtype {got.dtype} != {dtype}"
+    assert_exact(got.reshape(-1)[_sample_index(got.size)], np.frombuffer(bytes.fromhex(sample), dtype), f"{what} (sampled values)")
+    assert hashlib.sha256(got.tobytes()).hexdigest() == sha, f"{what}: the sampled values agree, but not all {got.size} values (sha256 differs)"
+
+
 def warp_cases():
+    """The warped image and mask of case i are stored with pack() under img_<i> / mask_<i> of `g`; the sources are drawn
+    again from the generator's seed (tests/golden/gen_golden.py gen_warp) and checked against the recorded sha256."""
     g = load("golden_warp.npz")
     from stitching_b200 import rigs
 
-    for i in range(int(g["n"])):
+    rng = np.random.default_rng(20260922)
+    srcs = [rng.integers(0, 256, (72, 96, 3), dtype=np.uint8) for _ in range(int(g["n"]))]
+    h = hashlib.sha256()
+    for src in srcs:
+        h.update(src.tobytes())
+    assert h.hexdigest() == str(g["src_sha256"]), "the seeded warp sources drifted from the goldens"
+    for i, src in enumerate(srcs):
         f, a, px, py = g[f"cam_{i}"]
         cam = rigs.Camera(f, a, px, py, g[f"R_{i}"])
         yield dict(i=i, wtype=str(g[f"type_{i}"]), cam=cam, scale=float(g[f"scale_{i}"]), aspect=float(g[f"aspect_{i}"]),
-                   src=g[f"src_{i}"], roi=tuple(int(v) for v in g[f"roi_{i}"]), img=g[f"img_{i}"], mask=g[f"mask_{i}"])
+                   src=src, roi=tuple(int(v) for v in g[f"roi_{i}"]), g=g)
 
 
 def blend_cases():
@@ -64,7 +107,7 @@ def e2e_cases():
             h.update(im.tobytes())
         assert h.hexdigest() == str(g[f"{name}_input_sha256"]), "synthetic input generator drifted from the goldens"
         yield dict(name=name, cfg=cfg, cams=cams, imgs=imgs, corners=[tuple(int(v) for v in r) for r in g[f"{name}_corners"]],
-                   sizes=[tuple(int(v) for v in r) for r in g[f"{name}_sizes"]], pano=g[f"{name}_pano"], pmask=g[f"{name}_pmask"])
+                   sizes=[tuple(int(v) for v in r) for r in g[f"{name}_sizes"]], g=g)  # pano / pmask: <name>_pano, <name>_pmask (pack)
 
 
 def run_warper_goldens(WarperCls):
@@ -74,8 +117,8 @@ def run_warper_goldens(WarperCls):
         w.scale = c["scale"]
         size = (c["src"].shape[1], c["src"].shape[0])
         assert tuple(w.warp_roi(size, c["cam"], c["aspect"])) == c["roi"], f"warp case {c['i']} ({c['wtype']}): roi"
-        assert_exact(w.warp_image(c["src"], c["cam"], c["aspect"]), c["img"], f"warp case {c['i']} ({c['wtype']}) image")
-        assert_exact(w.create_and_warp_mask(size, c["cam"], c["aspect"]), c["mask"], f"warp case {c['i']} ({c['wtype']}) mask")
+        assert_golden(w.warp_image(c["src"], c["cam"], c["aspect"]), c["g"], f"img_{c['i']}", f"warp case {c['i']} ({c['wtype']}) image")
+        assert_golden(w.create_and_warp_mask(size, c["cam"], c["aspect"]), c["g"], f"mask_{c['i']}", f"warp case {c['i']} ({c['wtype']}) mask")
 
 
 def run_blender_goldens(BlenderCls):
@@ -106,8 +149,8 @@ def run_e2e_goldens(WarperCls, BlenderCls):
         for img, m, corner in zip(warped, masks, corners):
             b.feed(img, m, corner)
         pano, pmask = b.blend()
-        assert_exact(pano, c["pano"], f"{c['name']} pano")
-        assert_exact(pmask, c["pmask"], f"{c['name']} mask")
+        assert_golden(pano, c["g"], f"{c['name']}_pano", f"{c['name']} pano")
+        assert_golden(pmask, c["g"], f"{c['name']}_pmask", f"{c['name']} mask")
 
 
 class OracleWarper:

@@ -1,13 +1,18 @@
-"""Drop-in check against the real reference pipeline (build container only: needs /root/reference and cv2).
+"""Drop-in check against the real reference pipeline.
 
 stitching.Stitcher(crop=False) runs unmodified on three synthetic perspective views of a textured plane.  The
 reference's registration is not deterministic from run to run (RANSAC), so two whole runs cannot be compared;
-instead every call that crosses the hot-path boundary (Warper, SeamFinder.resize, Blender) is RECORDED while the reference runs with its own classes
-(the exact cv.detail.CameraParams, numpy-float aspect, cv.UMat blend masks, corner tuples it hands over, and what
-cv2 returned), and then REPLAYED through the B200 classes (here on the emulation build, tests/emu): every warped
-image, mask, roi and the final panorama must be identical.  A second part runs the whole pipeline with
-stitching_b200.install() to show that it executes end to end on the swapped classes.
+instead every call that crosses the hot-path boundary (Warper, SeamFinder.resize, Blender) was RECORDED while the reference ran with its
+own classes (the cameras, aspects, blend masks and corners it hands over, with the container type of every image argument, and
+what cv2 returned; stored in tests/golden/golden_dropin.npz, written by write_golden), and is REPLAYED through the B200 classes
+(here on the emulation build, tests/emu) with arguments of the same types: cv.detail.CameraParams rebuilt from the recorded
+focal, aspect, principal point and R, numpy-float aspects, cv.UMat where the pipeline passed cv.UMat.  Every warped image,
+mask, roi and the final panorama must be identical.  A second part
+runs the whole pipeline with stitching_b200.install() to show that it executes end to end on the swapped classes; it needs
+the reference package (OpenStitching/stitching): oracle/_ref, which build() compiles from a reference checkout, or an
+installed `stitching`.
 """
+import hashlib
 import importlib
 import os
 import sys
@@ -15,22 +20,34 @@ import sys
 import numpy as np
 import pytest
 
-REF = "/root/reference"
+import replay
+
+GOLDEN = "golden_dropin.npz"
 
 
 @pytest.fixture()
 def reference_stitching():
+    """The reference package, fresh for every test (install() patches it): from oracle/_ref, which build() compiles from a
+    reference checkout (oracle/reference.py), or else an installed `stitching`."""
+    from oracle import reference
+
     cv = pytest.importorskip("cv2")
-    if not os.path.isdir(os.path.join(REF, "stitching")):
-        pytest.skip("the reference checkout is not on this box")
-    sys.path.insert(0, REF)
+    ref_dir = reference.REF_DIR if os.path.isfile(os.path.join(reference.REF_DIR, "stitching", "__init__.pyc")) else None
+    if ref_dir:
+        sys.path.insert(0, ref_dir)
     for name in [m for m in sys.modules if m == "stitching" or m.startswith("stitching.")]:
         del sys.modules[name]
-    mod = importlib.import_module("stitching")
-    yield mod, cv
-    for name in [m for m in sys.modules if m == "stitching" or m.startswith("stitching.")]:
-        del sys.modules[name]
-    sys.path.remove(REF)
+    try:
+        if ref_dir:  # built here: it has to import (a .pyc of another Python version fails here instead of skipping)
+            yield importlib.import_module("stitching"), cv
+        else:
+            yield pytest.importorskip("stitching", reason="no reference package: neither oracle/_ref (build() with a reference "
+                                                          "checkout) nor an installed one"), cv
+    finally:
+        for name in [m for m in sys.modules if m == "stitching" or m.startswith("stitching.")]:
+            del sys.modules[name]
+        if ref_dir:
+            sys.path.remove(ref_dir)
 
 
 def synthetic_views(cv):
@@ -62,12 +79,10 @@ def synthetic_views(cv):
 SETTINGS = dict(crop=False, detector="orb", confidence_threshold=0.3)
 
 
-def test_recorded_boundary_calls_replay_identically(reference_stitching, use_emu):
-    stitching, cv = reference_stitching
+def record_boundary_calls(stitching, cv):
+    """Run stitching.Stitcher with its own classes and log every call that crosses the hot-path boundary."""
     from stitching.blender import Blender as RefBlender
     from stitching.warper import Warper as RefWarper
-
-    import stitching_b200
 
     log = []
 
@@ -148,46 +163,149 @@ def test_recorded_boundary_calls_replay_identically(reference_stitching, use_emu
     applied = [e for e in log if e[0] == "gain_apply"]
     assert len(applied) == 3 and any(not np.array_equal(e[2], e[3]) for e in applied), "stitcher.py:219-221 compensates every image"
     assert any(type(e[2]).__name__ == "UMat" for e in log if e[0] == "feed"), "the pipeline hands cv.UMat masks to feed"
+    return log
 
-    blender = None
-    checked = 0
-    for e in log:
+
+def _sha(arr):
+    return hashlib.sha256(np.ascontiguousarray(arr).tobytes()).hexdigest()
+
+
+def write_golden(stitching, cv):
+    """Store one recorded run in tests/golden/GOLDEN: per call its arguments and what the reference returned (replay.pack).
+    An image argument that the synthetic views or an earlier call's result already is, is stored as that name
+    ("view_<i>", "out_<k>"); the others (the LOW-resolution seam masks of the graph cut, the gains) are stored whole."""
+    views = synthetic_views(cv)
+    log = record_boundary_calls(stitching, cv)
+    known = {_sha(v): f"view_{i}" for i, v in enumerate(views)}
+    out = {"n": np.int64(len(log)), "views_sha256": np.array([_sha(v) for v in views])}
+
+    def arg(k, name, arr):
+        out[f"e{k}_{name}_type"] = "UMat" if isinstance(arr, cv.UMat) else "ndarray"
+        arr = np.asarray(arr.get() if isinstance(arr, cv.UMat) else arr)
+        src = known.get(_sha(arr))
+        if src is None:
+            out[f"e{k}_{name}"] = arr
+        else:
+            out[f"e{k}_{name}_from"] = src
+
+    def result(k, arr):
+        replay.pack(out, f"e{k}_out", arr)
+        known.setdefault(_sha(arr), f"out_{k}")
+
+    for k, e in enumerate(log):
+        out[f"e{k}_kind"] = e[0]
         if e[0] in ("warp_image", "warp_mask", "warp_roi"):
-            w = stitching_b200.Warper(e[1])
-            w.scale = e[2]
-            got = {"warp_image": w.warp_image, "warp_mask": w.create_and_warp_mask, "warp_roi": w.warp_roi}[e[0]](e[3], e[4], e[5])
-            if e[0] == "warp_roi":
-                assert tuple(got) == e[6]
+            cam = e[4]
+            out[f"e{k}_warper"], out[f"e{k}_scale"], out[f"e{k}_aspect"] = e[1], np.float64(e[2]), np.float64(e[5])
+            out[f"e{k}_camera"] = np.array([cam.focal, cam.aspect, cam.ppx, cam.ppy], np.float64)
+            out[f"e{k}_R"] = np.asarray(cam.R)
+            if e[0] == "warp_image":
+                arg(k, "img", e[3])
+                result(k, e[6])
             else:
-                assert got.shape == e[6].shape and np.array_equal(got, e[6]), f"{e[0]}: {int((got != e[6]).sum())} values differ"
+                out[f"e{k}_size"] = np.array(e[3], np.int64)
+                if e[0] == "warp_mask":
+                    result(k, e[6])
+                else:
+                    out[f"e{k}_out"] = np.array(e[6], np.int64)
+        elif e[0] == "img_resize":
+            arg(k, "img", e[1])
+            out[f"e{k}_size"] = np.array(e[2], np.int64)
+            result(k, e[3])
+        elif e[0] == "gain_apply":
+            out[f"e{k}_gain"] = e[1]
+            arg(k, "img", e[2])
+            result(k, e[3])
+        elif e[0] == "seam_resize":
+            arg(k, "seam", e[1])
+            arg(k, "mask", e[2])
+            out[f"e{k}_out_type"] = e[4]
+            result(k, e[3])
+        elif e[0] == "prepare":
+            out[f"e{k}_blender"], out[f"e{k}_strength"] = e[1], np.float64(e[2])
+            out[f"e{k}_corners"], out[f"e{k}_sizes"] = np.array(e[3], np.int64), np.array(e[4], np.int64)
+        elif e[0] == "feed":
+            arg(k, "img", e[1])
+            arg(k, "mask", e[2])
+            out[f"e{k}_corner"] = np.array(e[3], np.int64)
+        elif e[0] == "blend":
+            replay.pack(out, f"e{k}_out", e[1])
+            replay.pack(out, f"e{k}_mask", e[2])
+    np.savez_compressed(os.path.join(replay.GOLDEN, GOLDEN), **out)
+
+
+def test_recorded_boundary_calls_replay_identically(use_emu):
+    """The calls one reference run made (GOLDEN, written by write_golden) replayed through the B200 classes."""
+    cv = pytest.importorskip("cv2")
+    import stitching_b200
+
+    g = replay.load(GOLDEN)
+    views = synthetic_views(cv)
+    assert [_sha(v) for v in views] == [str(s) for s in g["views_sha256"]], "synthetic_views drifted from the recorded run"
+    results = {f"view_{i}": v for i, v in enumerate(views)}
+
+    def arg(k, name):
+        arr = results[str(g[f"e{k}_{name}_from"])] if f"e{k}_{name}_from" in g.files else g[f"e{k}_{name}"]
+        return cv.UMat(arr) if str(g[f"e{k}_{name}_type"]) == "UMat" else arr
+
+    def camera(k):
+        cam = cv.detail.CameraParams()
+        cam.focal, cam.aspect, cam.ppx, cam.ppy = (float(v) for v in g[f"e{k}_camera"])
+        cam.R = g[f"e{k}_R"]
+        return cam
+
+    kinds = [str(g[f"e{k}_kind"]) for k in range(int(g["n"]))]
+    assert kinds.count("warp_image") >= 6 and kinds.count("feed") == 3 and kinds.count("blend") == 1
+    assert kinds.count("seam_resize") == 3 and kinds.count("img_resize") >= 6 and kinds.count("gain_apply") == 3
+    assert any(str(g[f"e{k}_mask_type"]) == "UMat" for k, kind in enumerate(kinds) if kind == "feed"), "the pipeline hands cv.UMat masks to feed"
+    blender = None
+    checked = compensated = 0
+    for k, kind in enumerate(kinds):
+        what = f"call {k} ({kind})"
+        if kind in ("warp_image", "warp_mask", "warp_roi"):
+            w = stitching_b200.Warper(str(g[f"e{k}_warper"]))
+            w.scale = float(g[f"e{k}_scale"])
+            cam, aspect = camera(k), np.float64(g[f"e{k}_aspect"])  # the numpy float the pipeline hands over
+            if kind == "warp_roi":
+                assert tuple(w.warp_roi(tuple(int(v) for v in g[f"e{k}_size"]), cam, aspect)) == tuple(int(v) for v in g[f"e{k}_out"]), what
+            else:
+                got = w.warp_image(arg(k, "img"), cam, aspect) if kind == "warp_image" else \
+                    w.create_and_warp_mask(tuple(int(v) for v in g[f"e{k}_size"]), cam, aspect)
+                replay.assert_golden(got, g, f"e{k}_out", what)
+                results[f"out_{k}"] = got
             checked += 1
-        elif e[0] == "img_resize":  # images.py:120-123: the MEDIUM / LOW / FINAL resolution inputs
-            got = stitching_b200.images.resize_exact(e[1], e[2])
-            assert got.shape == e[3].shape and np.array_equal(got, e[3]), f"Images.resize: {int((got != e[3]).sum())} values differ"
+        elif kind == "img_resize":  # images.py:120-123: the MEDIUM / LOW / FINAL resolution inputs
+            got = stitching_b200.images.resize_exact(arg(k, "img"), tuple(int(v) for v in g[f"e{k}_size"]))
+            replay.assert_golden(got, g, f"e{k}_out", f"{what}: Images.resize")
+            results[f"out_{k}"] = got
             checked += 1
-        elif e[0] == "gain_apply":  # the default compensator (gain_blocks) with the gains its own feed() estimated
-            got = stitching_b200.exposure_error_compensator.apply_gain(e[2].copy(), e[1])
-            assert np.array_equal(got, e[3]), f"ExposureErrorCompensator.apply: {int((got != e[3]).sum())} values differ"
+        elif kind == "gain_apply":  # the default compensator (gain_blocks) with the gains its own feed() estimated
+            before = arg(k, "img")
+            got = stitching_b200.exposure_error_compensator.apply_gain(before.copy(), g[f"e{k}_gain"])
+            replay.assert_golden(got, g, f"e{k}_out", f"{what}: ExposureErrorCompensator.apply")
+            compensated += not np.array_equal(got, before)
+            results[f"out_{k}"] = got
             checked += 1
-        elif e[0] == "seam_resize":  # the LOW-resolution seam mask arrives as cv.UMat, the warped mask as ndarray
-            got = stitching_b200.seam_finder.resize(e[1], e[2])
+        elif kind == "seam_resize":  # the LOW-resolution seam mask arrives as cv.UMat, the warped mask as ndarray
+            got = stitching_b200.seam_finder.resize(arg(k, "seam"), arg(k, "mask"))
             # same container type as the reference's cv2 chain (cv.UMat in the pipeline): seam_finder.py:47 and
             # verbose.py:149-156 call cv.UMat.get on it
-            assert type(got).__name__ == e[4], f"SeamFinder.resize returned {type(got).__name__}, the reference {e[4]}"
+            assert type(got).__name__ == str(g[f"e{k}_out_type"]), f"SeamFinder.resize returned {type(got).__name__}, the reference {g[f'e{k}_out_type']}"
             got = got.get() if hasattr(got, "get") else got
-            assert got.shape == e[3].shape and np.array_equal(got, e[3]), f"SeamFinder.resize: {int((got != e[3]).sum())} values differ"
+            replay.assert_golden(got, g, f"e{k}_out", f"{what}: SeamFinder.resize")
+            results[f"out_{k}"] = got
             checked += 1
-        elif e[0] == "prepare":
-            blender = stitching_b200.Blender(e[1], e[2])
-            blender.prepare(e[3], e[4])
-        elif e[0] == "feed":
-            blender.feed(e[1], e[2], e[3])
-        elif e[0] == "blend":
+        elif kind == "prepare":
+            blender = stitching_b200.Blender(str(g[f"e{k}_blender"]), float(g[f"e{k}_strength"]))
+            blender.prepare([tuple(int(v) for v in c) for c in g[f"e{k}_corners"]], [tuple(int(v) for v in s) for s in g[f"e{k}_sizes"]])
+        elif kind == "feed":
+            blender.feed(arg(k, "img"), arg(k, "mask"), tuple(int(v) for v in g[f"e{k}_corner"]))
+        elif kind == "blend":
             pano, mask = blender.blend()
-            assert np.array_equal(mask, e[2]) and pano.shape == e[1].shape
-            d = np.abs(pano.astype(np.int32) - e[1].astype(np.int32))
-            assert d.max() == 0, f"panorama: max |diff| {int(d.max())}, {int((d != 0).sum())} values"
+            replay.assert_golden(mask, g, f"e{k}_mask", "panorama mask")
+            replay.assert_golden(pano, g, f"e{k}_out", "panorama")
             checked += 1
+    assert compensated > 0, "stitcher.py:219-221 compensates every image"
     assert checked >= 19
 
 
@@ -294,3 +412,11 @@ def test_one_stitcher_for_two_image_sets_and_affine_stitcher_after_install(refer
         pytest.skip(f"the reference could not register the synthetic scans: {e}")
     assert pano.ndim == 3 and pano.dtype == np.uint8
     assert pano.shape[1] > 1200 and (pano.sum(axis=2) > 0).mean() > 0.5  # wider than one scan: the scans were composed
+
+
+if __name__ == "__main__":  # PYTHONPATH=.:tests:<reference checkout> python tests/test_dropin_pipeline.py
+    import cv2
+
+    import stitching
+
+    write_golden(stitching, cv2)
