@@ -94,6 +94,25 @@ SB_API int sb_resize_exact(const uint8_t *src, size_t src_pitch, int sw, int sh,
 SB_API int sb_seam_resize(const uint8_t *seam, size_t seam_pitch, int sw, int sh, const uint8_t *mask, size_t mask_pitch,
                           int w, int h, uint8_t *dst, size_t dst_pitch);
 
+/* ---------------------------------------------------------------------------------------------
+ * Pixel formats of frames going in and out of the compositor.  A YUV 4:2:0 frame (BT.601, limited range, what cameras,
+ * NVDEC / NVENC and ffmpeg's yuv420p carry) is given as up to three planes with a row pitch in bytes each:
+ *   SB_PIX_BGR   planes[0] = uint8 h x w x 3 (planes[1], planes[2] unused)
+ *   SB_PIX_NV12  planes[0] = Y, h rows of w bytes; planes[1] = interleaved U V, h/2 rows of w bytes
+ *   SB_PIX_I420  planes[0] = Y; planes[1] = U and planes[2] = V, h/2 rows of w/2 bytes each
+ * A YUV input frame means cv.cvtColor(frame, COLOR_YUV2BGR_NV12 / _I420) followed by the BGR pipeline; a YUV panorama
+ * means cv.cvtColor(pano, COLOR_BGR2YUV_I420) of the BGR panorama, with U and V interleaved for NV12.  Both are bit-exact
+ * to OpenCV.  As in OpenCV, YUV frames have even widths and heights (SB_ERR_INVALID otherwise).
+ * ------------------------------------------------------------------------------------------- */
+typedef enum { SB_PIX_BGR = 0, SB_PIX_NV12 = 1, SB_PIX_I420 = 2 } sb_pix_fmt;
+
+/* cv.cvtColor(COLOR_YUV2BGR_NV12 / _I420) with host buffers: fmt is SB_PIX_NV12 or SB_PIX_I420, dst uint8 h x w x 3 */
+SB_API int sb_cvt_yuv420_to_bgr(int fmt, const uint8_t *const planes[3], const size_t pitches[3], int w, int h, uint8_t *dst,
+                                size_t dst_pitch);
+/* cv.cvtColor(COLOR_BGR2YUV_I420) with host buffers, chroma interleaved for SB_PIX_NV12 */
+SB_API int sb_cvt_bgr_to_yuv420(int fmt, const uint8_t *src, size_t src_pitch, int w, int h, uint8_t *const planes[3],
+                                const size_t pitches[3]);
+
 /* warper.py:43-52 Warper.warp_image   -> PyRotationWarper.warp(INTER_LINEAR, BORDER_REFLECT)
  * warper.py:58-68 create_and_warp_mask -> PyRotationWarper.warp(INTER_NEAREST, BORDER_CONSTANT) on a 255 mask
  * Both outputs come from ONE kernel pass.  dst_img / dst_mask may each be NULL; their extents must be
@@ -191,6 +210,10 @@ SB_API int sb_compositor_model_bytes(const sb_compositor *c, double *total_bytes
 /* host -> device copy of source image i (uint8 HxWx3); asynchronous on the compositor stream when
  * `pinned` != 0 (caller guarantees page-locked memory and keeps it alive until sync) */
 SB_API int sb_compositor_upload(sb_compositor *c, int i, const uint8_t *src, size_t pitch, int pinned);
+/* the same for a frame in any sb_pix_fmt (sb_compositor_upload is this with SB_PIX_BGR); a YUV frame is converted on the
+ * device.  YUV frames need a single-GPU compositor (SB_ERR_STATE on a sharded one). */
+SB_API int sb_compositor_upload_frame(sb_compositor *c, int i, int fmt, const uint8_t *const planes[3], const size_t pitches[3],
+                                      int pinned);
 /* optional per-image blend mask in warped coordinates (mask_mode 1), uint8 h' x w' */
 SB_API int sb_compositor_set_mask(sb_compositor *c, int i, const uint8_t *mask, size_t pitch);
 /* the same from the LOW-resolution seam mask of image i (uint8 sh x sw, what SeamFinder.find returns): the device
@@ -205,12 +228,23 @@ SB_API int sb_compositor_set_gain(sb_compositor *c, int i, const float *gain_map
 SB_API int sb_compositor_run(sb_compositor *c);
 /* device -> host copy of the panorama (uint8 HxWx3 + uint8 mask); synchronises */
 SB_API int sb_compositor_download(sb_compositor *c, uint8_t *dst, size_t dst_pitch, uint8_t *dst_mask, size_t mask_pitch);
+/* the same with the panorama in any sb_pix_fmt (sb_compositor_download is this with SB_PIX_BGR); planes == NULL or
+ * planes[0] == NULL skips the panorama, dst_mask == NULL the mask.  A YUV panorama needs an even panorama size and a
+ * single-GPU compositor (SB_ERR_STATE on a sharded one). */
+SB_API int sb_compositor_download_frame(sb_compositor *c, int fmt, uint8_t *const planes[3], const size_t pitches[3], uint8_t *dst_mask,
+                                        size_t mask_pitch);
 /* Pipelined end-to-end step (throughput path): enqueue H2D of the n sources, warp + blend, and D2H of the
  * panorama on separate streams chained by events, and return a ticket.  Three buffer sets are kept, so at most
  * three tickets may be in flight: the copies of one step overlap the kernels of its neighbours.  Host buffers
  * should be page-locked (sb_host_alloc) and must stay valid until sb_compositor_wait(ticket) returns. */
 SB_API int sb_compositor_submit(sb_compositor *c, const uint8_t *const *srcs, const size_t *pitches, uint8_t *dst,
                                 size_t dst_pitch, uint8_t *dst_mask, size_t mask_pitch, unsigned long long *ticket);
+/* the same with sources and panorama in any sb_pix_fmt (sb_compositor_submit is this with SB_PIX_BGR both ways): planes /
+ * pitches hold three entries per source image (planes[3 i + k]), out_planes == NULL or out_planes[0] == NULL skips the
+ * panorama.  The YUV copies share the copy streams with the BGR ones; the conversions run on the device. */
+SB_API int sb_compositor_submit_frames(sb_compositor *c, int in_fmt, const uint8_t *const *planes, const size_t *pitches, int out_fmt,
+                                       uint8_t *const out_planes[3], const size_t out_pitches[3], uint8_t *dst_mask, size_t mask_pitch,
+                                       unsigned long long *ticket);
 SB_API int sb_compositor_wait(sb_compositor *c, unsigned long long ticket);
 /* device -> host copy of warped image i / its mask (for parity tests of the fused path) */
 SB_API int sb_compositor_download_warped(sb_compositor *c, int i, uint8_t *dst, size_t dst_pitch, uint8_t *dst_mask,

@@ -20,6 +20,7 @@ WARP_TYPES = {  # warper.py:10-27 -> sb_warp_type
     "mercator": 14, "transverseMercator": 15,
 }
 BLEND_KINDS = {"no": 0, "feather": 1, "multiband": 2}
+PIX_FMTS = {"bgr": 0, "nv12": 1, "i420": 2}  # sb_pix_fmt
 
 c_float_p = C.POINTER(C.c_float)
 c_int_p = C.POINTER(C.c_int)
@@ -72,6 +73,13 @@ SIGNATURES = [
     ("sb_compositor_geometry", C.c_int, [C.c_void_p, c_int_p, c_int_p, c_int_p]),
     ("sb_compositor_model_bytes", C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_int]),
     ("sb_compositor_upload", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_int]),
+    ("sb_compositor_upload_frame", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int]),
+    ("sb_compositor_download_frame", C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_void_p, C.c_size_t]),
+    ("sb_compositor_submit_frames", C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int,
+                                              C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_void_p, C.c_size_t,
+                                              C.POINTER(C.c_ulonglong)]),
+    ("sb_cvt_yuv420_to_bgr", C.c_int, [C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int, C.c_int, C.c_void_p, C.c_size_t]),
+    ("sb_cvt_bgr_to_yuv420", C.c_int, [C.c_int, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]),
     ("sb_compositor_set_mask", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]),
     ("sb_compositor_set_seam_mask", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_int, C.c_int]),
     ("sb_compositor_set_gain", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),

@@ -10,7 +10,7 @@ from statistics import median
 
 import numpy as np
 
-from . import _lib
+from . import _lib, color
 from .stitching_error import StitchingError
 from .warper import Warper
 
@@ -73,11 +73,20 @@ class Compositor:
         self.strip_axis = int(L.sb_compositor_shard_axis(self._c))  # 0: self.strip are columns of the panorama, 1: rows
 
     # -- data movement ---------------------------------------------------------------------------
-    def upload(self, images, pinned=False):
-        """images: the frames of THIS rank's block, in order (all n frames when world == 1)."""
+    def upload(self, images, pinned=False, fmt="bgr"):
+        """images: the frames of THIS rank's block, in order (all n frames when world == 1).
+
+        fmt "nv12" / "i420": YUV 4:2:0 frames as (h * 3/2, w) uint8 arrays (stitching_b200.color), converted to BGR on the
+        device exactly as cv.cvtColor does (single-GPU compositors, even frame sizes)."""
         L = _lib.lib()
         if len(images) != self.count:
             raise StitchingError(f"expected {self.count} images (block {self.first}..{self.first + self.count - 1}), got {len(images)}")
+        if fmt != "bgr":
+            code = color.fmt_code(fmt)
+            for i, img in enumerate(images, start=self.first):
+                ptrs, pitches, _keep = color.planes(img, self.sizes[i][0], self.sizes[i][1], fmt)
+                _lib.check(L.sb_compositor_upload_frame(self._c, i, code, ptrs, pitches, int(pinned)), "sb_compositor_upload_frame")
+            return
         for i, img in enumerate(images, start=self.first):
             img = np.asarray(img)
             if img.dtype != np.uint8 or img.shape != (self.sizes[i][1], self.sizes[i][0], 3):
@@ -126,13 +135,24 @@ class Compositor:
     def sync(self):
         _lib.check(_lib.lib().sb_compositor_sync(self._c), "sb_compositor_sync")
 
-    def download(self, out=None, out_mask=None):
-        """(pano, mask); with world > 1 the columns (strip_axis 0) or rows (strip_axis 1) self.strip[0]:self.strip[1]."""
+    def download(self, out=None, out_mask=None, fmt="bgr"):
+        """(pano, mask); with world > 1 the columns (strip_axis 0) or rows (strip_axis 1) self.strip[0]:self.strip[1].
+
+        fmt "nv12" / "i420": the panorama as a (h * 3/2, w) YUV 4:2:0 array, cv.cvtColor(pano, COLOR_BGR2YUV_I420) of the BGR
+        panorama (U and V interleaved for nv12), converted on the device (single-GPU compositors, even panorama sizes)."""
         h, w = self.roi[3], self.roi[2]
         if self.strip_axis == 0:
             w = self.strip[1] - self.strip[0]
         else:
             h = self.strip[1] - self.strip[0]
+        if fmt != "bgr":
+            pano = np.empty(color.frame_shape(w, h, fmt), np.uint8) if out is None else out
+            mask = np.empty((h, w), np.uint8) if out_mask is None else out_mask
+            ptrs, pitches, _ = color.planes(pano, w, h, fmt, writable=True)
+            _lib.check(_lib.lib().sb_compositor_download_frame(self._c, color.fmt_code(fmt), ptrs, pitches,
+                                                               mask.ctypes.data_as(C.c_void_p), mask.strides[0]),
+                       "sb_compositor_download_frame")
+            return pano, mask
         pano = np.empty((h, w, 3), np.uint8) if out is None else out
         mask = np.empty((h, w), np.uint8) if out_mask is None else out_mask
         _lib.check(_lib.lib().sb_compositor_download(self._c, pano.ctypes.data_as(C.c_void_p), pano.strides[0],
@@ -161,10 +181,15 @@ class Compositor:
                    "sb_compositor_shard_slab")
         return p.value, n.value
 
-    def submit(self, images, out, out_mask):
+    def submit(self, images, out, out_mask, in_fmt="bgr", out_fmt="bgr"):
         """Pipelined step: enqueue upload of `images`, warp + blend, download into `out` / `out_mask`; returns a
         ticket for wait().  At most three tickets in flight; host arrays should live in pinned memory
-        (`pinned_empty`) and must stay untouched until wait(ticket) returns."""
+        (`pinned_empty`) and must stay untouched until wait(ticket) returns.
+
+        in_fmt / out_fmt "nv12" / "i420": sources and / or panorama as (h * 3/2, w) YUV 4:2:0 arrays (see upload and
+        download); with YUV formats `out` and `out_mask` may be None (that output is not copied back)."""
+        if in_fmt != "bgr" or out_fmt != "bgr":
+            return self._submit_frames(images, out, out_mask, in_fmt, out_fmt)
         n = self.n
         ptrs = (C.c_void_p * n)()
         pitches = (C.c_size_t * n)()
@@ -179,6 +204,32 @@ class Compositor:
                    "sb_compositor_submit")
         return ticket.value
 
+    def _submit_frames(self, images, out, out_mask, in_fmt, out_fmt):
+        n = self.n
+        if len(images) != n:
+            raise StitchingError(f"expected {n} images, got {len(images)}")
+        in_code, out_code = color.fmt_code(in_fmt), color.fmt_code(out_fmt)
+        ptrs = (C.c_void_p * (3 * n))()
+        pitches = (C.c_size_t * (3 * n))()
+        for i, img in enumerate(images):
+            if not isinstance(img, np.ndarray):
+                raise StitchingError(f"image {i}: expected a uint8 ndarray")
+            p, q, arr = color.planes(img, self.sizes[i][0], self.sizes[i][1], in_fmt)
+            if arr is not img:  # a copy would not outlive this call: the caller's array must already have the layout
+                raise StitchingError(f"image {i}: the {in_fmt} frame must be laid out like a C-contiguous array")
+            ptrs[3 * i: 3 * i + 3] = list(p)
+            pitches[3 * i: 3 * i + 3] = list(q)
+        _, _, pw, ph = self.roi
+        out_ptrs, out_pitches = (C.c_void_p * 3)(), (C.c_size_t * 3)()
+        if out is not None:
+            out_ptrs, out_pitches, _ = color.planes(out, pw, ph, out_fmt, writable=True)
+        ticket = C.c_ulonglong()
+        _lib.check(_lib.lib().sb_compositor_submit_frames(self._c, in_code, ptrs, pitches, out_code, out_ptrs, out_pitches,
+                                                          None if out_mask is None else out_mask.ctypes.data_as(C.c_void_p),
+                                                          0 if out_mask is None else out_mask.strides[0], C.byref(ticket)),
+                   "sb_compositor_submit_frames")
+        return ticket.value
+
     def wait(self, ticket):
         _lib.check(_lib.lib().sb_compositor_wait(self._c, C.c_ulonglong(ticket)), "sb_compositor_wait")
 
@@ -191,11 +242,12 @@ class Compositor:
         self._pinned.append(p)
         return np.ctypeslib.as_array((C.c_uint8 * nbytes).from_address(p)).reshape(shape)
 
-    def composite(self, images):
-        """One call: upload, warp + blend, download.  Returns (uint8 pano, uint8 mask) like Blender.blend()."""
-        self.upload(images)
+    def composite(self, images, in_fmt="bgr", out_fmt="bgr"):
+        """One call: upload, warp + blend, download.  Returns (uint8 pano, uint8 mask) like Blender.blend(); the pixel
+        formats are those of upload and download."""
+        self.upload(images, fmt=in_fmt)
         self.run()
-        return self.download()
+        return self.download(fmt=out_fmt)
 
     # -- measurement -------------------------------------------------------------------------------
     def time(self, iters, flush_l2=False):

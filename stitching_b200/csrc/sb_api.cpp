@@ -484,6 +484,62 @@ int sb_seam_resize(const uint8_t *seam, size_t seam_pitch, int sw, int sh, const
 }
 
 // -------------------------------------------------------------------------------------------------
+// cv.cvtColor between BGR and YUV 4:2:0 (sb_yuv.cu) with host buffers
+// -------------------------------------------------------------------------------------------------
+static int check_yuv_size(const char *who, int fmt, int w, int h)
+{
+    if (fmt != SB_PIX_NV12 && fmt != SB_PIX_I420) {
+        set_error("%s: format %d is not a YUV 4:2:0 format (SB_PIX_NV12, SB_PIX_I420)", who, fmt);
+        return SB_ERR_INVALID;
+    }
+    if (w <= 0 || h <= 0 || (w | h) & 1 || (long long)w * h > (1ll << 31)) {
+        set_error("%s: a YUV 4:2:0 frame needs an even width and height, got %dx%d", who, w, h);
+        return SB_ERR_INVALID;
+    }
+    return SB_OK;
+}
+
+int sb_cvt_yuv420_to_bgr(int fmt, const uint8_t *const planes[3], const size_t pitches[3], int w, int h, uint8_t *dst, size_t dst_pitch)
+{
+    SB_TRY(check_yuv_size("sb_cvt_yuv420_to_bgr", fmt, w, h));
+    if (!yuv_planes_ok(fmt, planes, pitches, w) || !dst || dst_pitch < (size_t)w * 3) {
+        set_error("sb_cvt_yuv420_to_bgr: missing plane or short pitch");
+        return SB_ERR_INVALID;
+    }
+    SB_TRY(ensure_device());
+    cudaStream_t s = default_stream();
+    Scratch tmp(s);
+    uint8_t *d_yuv = nullptr, *d_bgr = nullptr;
+    SB_TRY(tmp.get(&d_yuv, yuv_bytes(w, h)));
+    SB_TRY(tmp.get(&d_bgr, (size_t)w * 3 * h));
+    SB_CUDA(yuv_copy(d_yuv, planes, pitches, fmt, w, h, cudaMemcpyHostToDevice, s));
+    SB_TRY(launch_yuv420_to_src(fmt, yuv_dense_planes(fmt, d_yuv, w, h), w, h, d_bgr, (long long)w * 3, nullptr, 0, s));
+    SB_CUDA(sb_copy2d(dst, dst_pitch, d_bgr, (size_t)w * 3, (size_t)w * 3, h, cudaMemcpyDeviceToHost, s));
+    SB_CUDA(cudaStreamSynchronize(s));
+    return SB_OK;
+}
+
+int sb_cvt_bgr_to_yuv420(int fmt, const uint8_t *src, size_t src_pitch, int w, int h, uint8_t *const planes[3], const size_t pitches[3])
+{
+    SB_TRY(check_yuv_size("sb_cvt_bgr_to_yuv420", fmt, w, h));
+    if (!yuv_planes_ok(fmt, planes, pitches, w) || !src || src_pitch < (size_t)w * 3) {
+        set_error("sb_cvt_bgr_to_yuv420: missing plane or short pitch");
+        return SB_ERR_INVALID;
+    }
+    SB_TRY(ensure_device());
+    cudaStream_t s = default_stream();
+    Scratch tmp(s);
+    uint8_t *d_yuv = nullptr, *d_bgr = nullptr;
+    SB_TRY(tmp.get(&d_yuv, yuv_bytes(w, h)));
+    SB_TRY(tmp.get(&d_bgr, (size_t)w * 3 * h));
+    SB_CUDA(sb_copy2d(d_bgr, (size_t)w * 3, src, src_pitch, (size_t)w * 3, h, cudaMemcpyHostToDevice, s));
+    SB_TRY(launch_bgr_to_yuv420(fmt, d_bgr, (long long)w * 3, w, h, yuv_dense_out(fmt, d_yuv, w, h), s));
+    SB_CUDA(yuv_copy(d_yuv, planes, pitches, fmt, w, h, cudaMemcpyDeviceToHost, s));
+    SB_CUDA(cudaStreamSynchronize(s));
+    return SB_OK;
+}
+
+// -------------------------------------------------------------------------------------------------
 // Blender
 // -------------------------------------------------------------------------------------------------
 struct sb_blender {

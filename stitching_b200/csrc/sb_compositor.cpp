@@ -36,6 +36,12 @@ struct sb_compositor {
     std::vector<uint32_t *> src4_dev;  // the same, one word per pixel: what the warp kernel reads (repacked after every upload)
     std::vector<uint32_t *> src4_devx[SB_PIPE_DEPTH - 1];
     bool use_src4 = true;
+    // YUV frames (sb_pix_fmt): src4_only[i] when the warp kernel reads image i's word-per-pixel source and never the 3-byte
+    // one, which then stages the YUV upload (3 B/px >= 1.5 B/px); otherwise the YUV frame has a staging buffer of its own
+    // per buffer slot.  yuv_out: the YUV panorama of each slot.  All allocated on first use.
+    std::vector<char> src4_only;
+    std::vector<uint8_t *> yuv_in[SB_PIPE_DEPTH];
+    uint8_t *yuv_out[SB_PIPE_DEPTH] = {};
     std::vector<uint32_t *> rgbm_dev;  // warped, packed; row pitch = width rounded up to 32 pixels (128-byte rows)
     std::vector<float *> tab_dev;
     std::vector<float *> maps_dev;     // projections that are not separable: xmap | ymap of every image (built at plan time)
@@ -80,6 +86,11 @@ static void compositor_free(sb_compositor *c)
     for (auto p : c->src4_dev) dev_free(p, s);
     for (auto &v : c->src4_devx)
         for (auto p : v) dev_free(p, s);
+    if (c->h2d) (void)cudaStreamSynchronize(c->h2d);
+    if (c->d2h) (void)cudaStreamSynchronize(c->d2h);
+    for (auto &v : c->yuv_in)
+        for (auto p : v) dev_free(p, s);
+    for (auto p : c->yuv_out) dev_free(p, s);
     for (auto p : c->rgbm_dev) dev_free(p, s);
     for (auto p : c->tab_dev) dev_free(p, s);
     for (auto p : c->maps_dev) dev_free(p, s);
@@ -202,6 +213,9 @@ static int compositor_build(sb_compositor *c, const sb_rig *rig, int rank, int w
         c->jobs[i].rgbm_pitch = rgbm_pitch_of(rect[2]);
         c->warp_bytes += 3.0 * c->src_w[i] * c->src_h[i] + 4.0 * rect[2] * rect[3];
     }
+    c->src4_only.assign(n, 0);
+    for (int i = c->first; i < c->first + c->count; ++i)
+        c->src4_only[i] = warp_reads_src4_only(c->jobs.data() + c->first, c->count, i - c->first);
 
     // Blender.prepare (blender.py:23-38)
     const Rect roi = result_roi(corners.data(), sizes.data(), n);
@@ -497,6 +511,218 @@ static int compositor_pipe_init(sb_compositor *c)
     return SB_OK;
 }
 
+// ---- frames in other pixel formats (sb_pix_fmt) ----------------------------------------------------------------------
+static bool valid_fmt(int fmt) { return fmt == SB_PIX_BGR || fmt == SB_PIX_NV12 || fmt == SB_PIX_I420; }
+
+static uint8_t *src_of(sb_compositor *c, int slot, int i) { return slot ? c->src_devx[slot - 1][i] : c->src_dev[i]; }
+static uint32_t *src4_of(sb_compositor *c, int slot, int i)
+{
+    return slot ? (c->src4_devx[slot - 1].empty() ? nullptr : c->src4_devx[slot - 1][i]) : c->src4_dev[i];
+}
+static uint8_t *yuv_stage_of(sb_compositor *c, int slot, int i) { return c->src4_only[i] ? src_of(c, slot, i) : c->yuv_in[slot][i]; }
+
+// the buffers a YUV step of `slot` needs (sources staged when in_fmt is YUV, the panorama when out_fmt is YUV), allocated
+// on first use; synchronises the compute stream after an allocation, so that any stream may use them next
+static int yuv_buffers(sb_compositor *c, int slot, int in_fmt, int out_fmt)
+{
+    cudaStream_t s = c->stream;
+    bool allocated = false;
+    if (in_fmt != SB_PIX_BGR) {
+        auto &v = c->yuv_in[slot];
+        if (v.empty()) v.assign(c->n, nullptr);
+        for (int i = 0; i < c->n; ++i)
+            if (!c->src4_only[i] && !v[i]) {
+                SB_TRY(dev_alloc((void **)&v[i], yuv_bytes(c->src_w[i], c->src_h[i]), s));
+                allocated = true;
+            }
+    }
+    if (out_fmt != SB_PIX_BGR && !c->yuv_out[slot]) {
+        SB_TRY(dev_alloc((void **)&c->yuv_out[slot], yuv_bytes(c->out.w, c->out.h), s));
+        allocated = true;
+    }
+    if (allocated) SB_CUDA(cudaStreamSynchronize(s));
+    return SB_OK;
+}
+
+// cv.cvtColor(COLOR_YUV2BGR_*) of the staged frame of image i into exactly the source the warp kernel reads
+static int yuv_convert_source(sb_compositor *c, int slot, int i, int fmt, cudaStream_t s)
+{
+    const int w = c->src_w[i], h = c->src_h[i];
+    const YuvPlanes in = yuv_dense_planes(fmt, yuv_stage_of(c, slot, i), w, h);
+    if (c->src4_only[i]) return launch_yuv420_to_src(fmt, in, w, h, nullptr, 0, src4_of(c, slot, i), w, s);
+    return launch_yuv420_to_src(fmt, in, w, h, src_of(c, slot, i), (long long)w * 3, nullptr, 0, s);
+}
+
+// the checks a YUV frame of the panorama (is_out) or of source image i has to pass
+static int yuv_frame_ok(const sb_compositor *c, const char *who, int fmt, bool is_out, int i)
+{
+    if (fmt == SB_PIX_BGR) return SB_OK;
+    if (c->sharded) {
+        set_error("%s: YUV frames need a single-GPU compositor", who);
+        return SB_ERR_STATE;
+    }
+    const int w = is_out ? c->out.w : c->src_w[i], h = is_out ? c->out.h : c->src_h[i];
+    if ((w | h) & 1) {
+        if (is_out)
+            set_error("%s: a YUV 4:2:0 panorama needs an even width and height, the panorama is %dx%d", who, w, h);
+        else
+            set_error("%s: a YUV 4:2:0 frame needs an even width and height, image %d is %dx%d", who, i, w, h);
+        return SB_ERR_INVALID;
+    }
+    return SB_OK;
+}
+
+static int upload_frame(sb_compositor *c, int i, int fmt, const uint8_t *const planes[3], const size_t pitches[3], int pinned,
+                        const char *who)
+{
+    if (!c || i < 0 || i >= c->n || !valid_fmt(fmt) || !planes || !pitches) {
+        set_error("%s: invalid argument", who);
+        return SB_ERR_INVALID;
+    }
+    if (fmt == SB_PIX_BGR) {
+        const uint8_t *src = planes[0];
+        const size_t pitch = pitches[0];
+        if (!src || pitch < (size_t)c->src_w[i] * 3) {
+            set_error("%s: invalid argument", who);
+            return SB_ERR_INVALID;
+        }
+        if (!c->src_dev[i]) {
+            set_error("%s: image %d belongs to another rank (this rank owns %d..%d)", who, i, c->first, c->first + c->count - 1);
+            return SB_ERR_INVALID;
+        }
+        SB_CUDA(sb_copy2d(c->src_dev[i], (size_t)c->src_w[i] * 3, src, pitch, (size_t)c->src_w[i] * 3, c->src_h[i],
+                          cudaMemcpyHostToDevice, c->stream));
+        if (c->src4_dev[i]) SB_TRY(launch_repack_rgbx(c->src_dev[i], c->src4_dev[i], (long long)c->src_w[i] * c->src_h[i], c->stream));
+    } else {
+        SB_TRY(yuv_frame_ok(c, who, fmt, false, i));
+        if (!yuv_planes_ok(fmt, planes, pitches, c->src_w[i])) {
+            set_error("%s: image %d: missing plane or short pitch", who, i);
+            return SB_ERR_INVALID;
+        }
+        SB_TRY(yuv_buffers(c, 0, fmt, SB_PIX_BGR));
+        SB_CUDA(yuv_copy(yuv_stage_of(c, 0, i), planes, pitches, fmt, c->src_w[i], c->src_h[i], cudaMemcpyHostToDevice, c->stream));
+        SB_TRY(yuv_convert_source(c, 0, i, fmt, c->stream));
+    }
+    if (!pinned) SB_CUDA(cudaStreamSynchronize(c->stream));
+    return SB_OK;
+}
+
+static int download_frame(sb_compositor *c, int fmt, uint8_t *const planes[3], const size_t pitches[3], uint8_t *dst_mask,
+                          size_t mask_pitch, const char *who)
+{
+    uint8_t *dst = planes ? planes[0] : nullptr;
+    if (!c || !valid_fmt(fmt) || (dst && !pitches) || (dst_mask && mask_pitch < (size_t)c->out.w) ||
+        (dst && fmt == SB_PIX_BGR && pitches[0] < (size_t)c->out.w * 3)) {
+        set_error("%s: invalid argument", who);
+        return SB_ERR_INVALID;
+    }
+    if (dst && fmt != SB_PIX_BGR) {
+        SB_TRY(yuv_frame_ok(c, who, fmt, true, 0));
+        if (!yuv_planes_ok(fmt, planes, pitches, c->out.w)) {
+            set_error("%s: missing plane or short pitch", who);
+            return SB_ERR_INVALID;
+        }
+        SB_TRY(yuv_buffers(c, 0, SB_PIX_BGR, fmt));
+        // slot 0's YUV panorama may still be on its way to the host from a submitted step
+        if (c->pipe_ready) SB_CUDA(cudaStreamWaitEvent(c->stream, c->e_d2h[0], 0));
+        SB_TRY(launch_bgr_to_yuv420(fmt, c->out.rgb, c->out.rgb_pitch, c->out.w, c->out.h, yuv_dense_out(fmt, c->yuv_out[0], c->out.w, c->out.h),
+                                    c->stream));
+        SB_CUDA(yuv_copy(c->yuv_out[0], planes, pitches, fmt, c->out.w, c->out.h, cudaMemcpyDeviceToHost, c->stream));
+    } else if (dst) {
+        SB_CUDA(sb_copy2d(dst, pitches[0], c->out.rgb, (size_t)c->out.rgb_pitch, (size_t)c->out.w * 3, c->out.h, cudaMemcpyDeviceToHost,
+                          c->stream));
+    }
+    if (dst_mask)
+        SB_CUDA(sb_copy2d(dst_mask, mask_pitch, c->out.mask, (size_t)c->out.mask_pitch, c->out.w, c->out.h,
+                                  cudaMemcpyDeviceToHost, c->stream));
+    SB_CUDA(cudaStreamSynchronize(c->stream));
+    return SB_OK;
+}
+
+// Pipelined end-to-end step: H2D of this batch, warp + blend, D2H of the panorama are enqueued on three
+// streams and chained with events; with three buffer sets the copies of a step overlap the kernels and copies of its neighbours.
+static int submit_frames(sb_compositor *c, int in_fmt, const uint8_t *const *planes, const size_t *pitches, int out_fmt,
+                         uint8_t *const out_planes[3], const size_t out_pitches[3], uint8_t *dst_mask, size_t mask_pitch,
+                         unsigned long long *ticket, const char *who)
+{
+    uint8_t *dst = out_planes ? out_planes[0] : nullptr;
+    if (!c || !valid_fmt(in_fmt) || !valid_fmt(out_fmt) || !planes || !pitches || (dst && !out_pitches) ||
+        (dst && out_fmt == SB_PIX_BGR && out_pitches[0] < (size_t)c->out.w * 3) || (dst_mask && mask_pitch < (size_t)c->out.w)) {
+        set_error("%s: invalid argument", who);
+        return SB_ERR_INVALID;
+    }
+    if (c->sharded) {
+        set_error("%s: the pipelined path is single-GPU; use upload / run / download on a sharded compositor", who);
+        return SB_ERR_STATE;
+    }
+    for (int i = 0; i < c->n; ++i) {
+        if (in_fmt == SB_PIX_BGR ? (!planes[3 * i] || pitches[3 * i] < (size_t)c->src_w[i] * 3) : false) {
+            set_error("%s: invalid source %d", who, i);
+            return SB_ERR_INVALID;
+        }
+        SB_TRY(yuv_frame_ok(c, who, in_fmt, false, i));
+        if (in_fmt != SB_PIX_BGR && !yuv_planes_ok(in_fmt, planes + 3 * i, pitches + 3 * i, c->src_w[i])) {
+            set_error("%s: invalid source %d: missing plane or short pitch", who, i);
+            return SB_ERR_INVALID;
+        }
+    }
+    if (dst && out_fmt != SB_PIX_BGR) {
+        SB_TRY(yuv_frame_ok(c, who, out_fmt, true, 0));
+        if (!yuv_planes_ok(out_fmt, out_planes, out_pitches, c->out.w)) {
+            set_error("%s: missing panorama plane or short pitch", who);
+            return SB_ERR_INVALID;
+        }
+    }
+    SB_TRY(compositor_pipe_init(c));
+    const unsigned long long t = c->submitted;
+    const int slot = (int)(t % SB_PIPE_DEPTH);
+    SB_TRY(yuv_buffers(c, slot, in_fmt, dst ? out_fmt : SB_PIX_BGR));
+    const PanoOut &o = slot ? c->outx[slot - 1] : c->out;
+    // sources of this slot are free once the previous compute that read them has finished; on a slot's first use
+    // that is whatever upload() / run() / sb_compositor_time() queued on the compute stream before this submit
+    // (download() is synchronous, so the output buffers need no such guard)
+    if (t < SB_PIPE_DEPTH) SB_CUDA(cudaEventRecord(c->e_comp[slot], c->stream));
+    SB_CUDA(cudaStreamWaitEvent(c->h2d, c->e_comp[slot], 0));
+    for (int i = 0; i < c->n; ++i) {
+        if (in_fmt == SB_PIX_BGR)
+            SB_CUDA(sb_copy2d(src_of(c, slot, i), (size_t)c->src_w[i] * 3, planes[3 * i], pitches[3 * i], (size_t)c->src_w[i] * 3, c->src_h[i],
+                              cudaMemcpyHostToDevice, c->h2d));
+        else
+            SB_CUDA(yuv_copy(yuv_stage_of(c, slot, i), planes + 3 * i, pitches + 3 * i, in_fmt, c->src_w[i], c->src_h[i],
+                             cudaMemcpyHostToDevice, c->h2d));
+    }
+    // the repack / conversion kernels follow the LAST copy (same stream): a kernel between two copies would leave the PCIe
+    // link idle for its launch + run time, eight times per step
+    for (int i = 0; i < c->n; ++i) {
+        if (in_fmt != SB_PIX_BGR) {
+            SB_TRY(yuv_convert_source(c, slot, i, in_fmt, c->h2d));
+            continue;
+        }
+        uint32_t *s4 = src4_of(c, slot, i);
+        if (s4) SB_TRY(launch_repack_rgbx(src_of(c, slot, i), s4, (long long)c->src_w[i] * c->src_h[i], c->h2d));
+    }
+    SB_CUDA(cudaEventRecord(c->e_h2d[slot], c->h2d));
+    SB_CUDA(cudaStreamWaitEvent(c->stream, c->e_h2d[slot], 0));
+    // the output buffers of this slot are free once their previous download has finished
+    if (t >= SB_PIPE_DEPTH) SB_CUDA(cudaStreamWaitEvent(c->stream, c->e_d2h[slot], 0));
+    SB_TRY(compositor_enqueue(c, false, slot));
+    const bool yuv_out = dst && out_fmt != SB_PIX_BGR;
+    if (yuv_out)  // after the step's graph, on the compute stream
+        SB_TRY(launch_bgr_to_yuv420(out_fmt, o.rgb, o.rgb_pitch, o.w, o.h, yuv_dense_out(out_fmt, c->yuv_out[slot], o.w, o.h), c->stream));
+    SB_CUDA(cudaEventRecord(c->e_comp[slot], c->stream));
+    SB_CUDA(cudaStreamWaitEvent(c->d2h, c->e_comp[slot], 0));
+    if (yuv_out)
+        SB_CUDA(yuv_copy(c->yuv_out[slot], out_planes, out_pitches, out_fmt, o.w, o.h, cudaMemcpyDeviceToHost, c->d2h));
+    else if (dst)
+        SB_CUDA(sb_copy2d(dst, out_pitches[0], o.rgb, (size_t)o.rgb_pitch, (size_t)o.w * 3, o.h, cudaMemcpyDeviceToHost, c->d2h));
+    if (dst_mask)
+        SB_CUDA(sb_copy2d(dst_mask, mask_pitch, o.mask, (size_t)o.mask_pitch, o.w, o.h, cudaMemcpyDeviceToHost, c->d2h));
+    SB_CUDA(cudaEventRecord(c->e_d2h[slot], c->d2h));
+    c->submitted = t + 1;
+    if (ticket) *ticket = t;
+    return SB_OK;
+}
+
 extern "C" {
 
 sb_compositor *sb_compositor_create(const sb_rig *rig)
@@ -628,19 +854,14 @@ int sb_compositor_model_bytes(const sb_compositor *c, double *total_bytes, doubl
 
 int sb_compositor_upload(sb_compositor *c, int i, const uint8_t *src, size_t pitch, int pinned)
 {
-    if (!c || i < 0 || i >= c->n || !src || pitch < (size_t)c->src_w[i] * 3) {
-        set_error("sb_compositor_upload: invalid argument");
-        return SB_ERR_INVALID;
-    }
-    if (!c->src_dev[i]) {
-        set_error("sb_compositor_upload: image %d belongs to another rank (this rank owns %d..%d)", i, c->first, c->first + c->count - 1);
-        return SB_ERR_INVALID;
-    }
-    SB_CUDA(sb_copy2d(c->src_dev[i], (size_t)c->src_w[i] * 3, src, pitch, (size_t)c->src_w[i] * 3, c->src_h[i],
-                              cudaMemcpyHostToDevice, c->stream));
-    if (c->src4_dev[i]) SB_TRY(launch_repack_rgbx(c->src_dev[i], c->src4_dev[i], (long long)c->src_w[i] * c->src_h[i], c->stream));
-    if (!pinned) SB_CUDA(cudaStreamSynchronize(c->stream));
-    return SB_OK;
+    const uint8_t *planes[3] = {src, nullptr, nullptr};
+    const size_t pitches[3] = {pitch, 0, 0};
+    return upload_frame(c, i, SB_PIX_BGR, planes, pitches, pinned, "sb_compositor_upload");
+}
+
+int sb_compositor_upload_frame(sb_compositor *c, int i, int fmt, const uint8_t *const planes[3], const size_t pitches[3], int pinned)
+{
+    return upload_frame(c, i, fmt, planes, pitches, pinned, "sb_compositor_upload_frame");
 }
 
 int sb_compositor_set_mask(sb_compositor *c, int i, const uint8_t *mask, size_t pitch)
@@ -761,72 +982,42 @@ int sb_compositor_sync(sb_compositor *c)
 
 int sb_compositor_download(sb_compositor *c, uint8_t *dst, size_t dst_pitch, uint8_t *dst_mask, size_t mask_pitch)
 {
-    if (!c || (dst && dst_pitch < (size_t)c->out.w * 3) || (dst_mask && mask_pitch < (size_t)c->out.w)) {
-        set_error("sb_compositor_download: invalid argument");
-        return SB_ERR_INVALID;
-    }
-    if (dst)
-        SB_CUDA(sb_copy2d(dst, dst_pitch, c->out.rgb, (size_t)c->out.rgb_pitch, (size_t)c->out.w * 3, c->out.h,
-                                  cudaMemcpyDeviceToHost, c->stream));
-    if (dst_mask)
-        SB_CUDA(sb_copy2d(dst_mask, mask_pitch, c->out.mask, (size_t)c->out.mask_pitch, c->out.w, c->out.h,
-                                  cudaMemcpyDeviceToHost, c->stream));
-    SB_CUDA(cudaStreamSynchronize(c->stream));
-    return SB_OK;
+    uint8_t *const planes[3] = {dst, nullptr, nullptr};
+    const size_t pitches[3] = {dst_pitch, 0, 0};
+    return download_frame(c, SB_PIX_BGR, planes, pitches, dst_mask, mask_pitch, "sb_compositor_download");
 }
 
-// Pipelined end-to-end step: H2D of this batch, warp + blend, D2H of the panorama are enqueued on three
-// streams and chained with events; with three buffer sets the copies of a step overlap the kernels and copies of its neighbours.
+int sb_compositor_download_frame(sb_compositor *c, int fmt, uint8_t *const planes[3], const size_t pitches[3], uint8_t *dst_mask,
+                                 size_t mask_pitch)
+{
+    return download_frame(c, fmt, planes, pitches, dst_mask, mask_pitch, "sb_compositor_download_frame");
+}
+
 int sb_compositor_submit(sb_compositor *c, const uint8_t *const *srcs, const size_t *pitches, uint8_t *dst, size_t dst_pitch,
                          uint8_t *dst_mask, size_t mask_pitch, unsigned long long *ticket)
 {
-    if (!c || !srcs || !pitches || (dst && dst_pitch < (size_t)c->out.w * 3) || (dst_mask && mask_pitch < (size_t)c->out.w)) {
-        set_error("sb_compositor_submit: invalid argument");
-        return SB_ERR_INVALID;
-    }
-    if (c->sharded) {
-        set_error("sb_compositor_submit: the pipelined path is single-GPU; use upload / run / download on a sharded compositor");
-        return SB_ERR_STATE;
-    }
-    for (int i = 0; i < c->n; ++i)
-        if (!srcs[i] || pitches[i] < (size_t)c->src_w[i] * 3) {
-            set_error("sb_compositor_submit: invalid source %d", i);
-            return SB_ERR_INVALID;
+    std::vector<const uint8_t *> planes;
+    std::vector<size_t> plane_pitches;
+    if (c && srcs && pitches) {  // one plane per source
+        planes.assign((size_t)3 * c->n, nullptr);
+        plane_pitches.assign((size_t)3 * c->n, 0);
+        for (int i = 0; i < c->n; ++i) {
+            planes[3 * i] = srcs[i];
+            plane_pitches[3 * i] = pitches[i];
         }
-    SB_TRY(compositor_pipe_init(c));
-    const unsigned long long t = c->submitted;
-    const int slot = (int)(t % SB_PIPE_DEPTH);
-    const std::vector<uint8_t *> &sdev = slot ? c->src_devx[slot - 1] : c->src_dev;
-    const PanoOut &o = slot ? c->outx[slot - 1] : c->out;
-    // sources of this slot are free once the previous compute that read them has finished; on a slot's first use
-    // that is whatever upload() / run() / sb_compositor_time() queued on the compute stream before this submit
-    // (download() is synchronous, so the output buffers need no such guard)
-    if (t < SB_PIPE_DEPTH) SB_CUDA(cudaEventRecord(c->e_comp[slot], c->stream));
-    SB_CUDA(cudaStreamWaitEvent(c->h2d, c->e_comp[slot], 0));
-    for (int i = 0; i < c->n; ++i)
-        SB_CUDA(sb_copy2d(sdev[i], (size_t)c->src_w[i] * 3, srcs[i], pitches[i], (size_t)c->src_w[i] * 3, c->src_h[i],
-                                  cudaMemcpyHostToDevice, c->h2d));
-    // the repack kernels follow the LAST copy (same stream): a kernel between two copies would leave the PCIe link idle
-    // for its launch + run time, eight times per step
-    for (int i = 0; i < c->n; ++i) {
-        uint32_t *s4 = slot ? (c->src4_devx[slot - 1].empty() ? nullptr : c->src4_devx[slot - 1][i]) : c->src4_dev[i];
-        if (s4) SB_TRY(launch_repack_rgbx(sdev[i], s4, (long long)c->src_w[i] * c->src_h[i], c->h2d));
     }
-    SB_CUDA(cudaEventRecord(c->e_h2d[slot], c->h2d));
-    SB_CUDA(cudaStreamWaitEvent(c->stream, c->e_h2d[slot], 0));
-    // the output buffers of this slot are free once their previous download has finished
-    if (t >= SB_PIPE_DEPTH) SB_CUDA(cudaStreamWaitEvent(c->stream, c->e_d2h[slot], 0));
-    SB_TRY(compositor_enqueue(c, false, slot));
-    SB_CUDA(cudaEventRecord(c->e_comp[slot], c->stream));
-    SB_CUDA(cudaStreamWaitEvent(c->d2h, c->e_comp[slot], 0));
-    if (dst)
-        SB_CUDA(sb_copy2d(dst, dst_pitch, o.rgb, (size_t)o.rgb_pitch, (size_t)o.w * 3, o.h, cudaMemcpyDeviceToHost, c->d2h));
-    if (dst_mask)
-        SB_CUDA(sb_copy2d(dst_mask, mask_pitch, o.mask, (size_t)o.mask_pitch, o.w, o.h, cudaMemcpyDeviceToHost, c->d2h));
-    SB_CUDA(cudaEventRecord(c->e_d2h[slot], c->d2h));
-    c->submitted = t + 1;
-    if (ticket) *ticket = t;
-    return SB_OK;
+    uint8_t *const out[3] = {dst, nullptr, nullptr};
+    const size_t out_pitches[3] = {dst_pitch, 0, 0};
+    return submit_frames(c, SB_PIX_BGR, planes.empty() ? nullptr : planes.data(), plane_pitches.empty() ? nullptr : plane_pitches.data(),
+                         SB_PIX_BGR, out, out_pitches, dst_mask, mask_pitch, ticket, "sb_compositor_submit");
+}
+
+int sb_compositor_submit_frames(sb_compositor *c, int in_fmt, const uint8_t *const *planes, const size_t *pitches, int out_fmt,
+                                uint8_t *const out_planes[3], const size_t out_pitches[3], uint8_t *dst_mask, size_t mask_pitch,
+                                unsigned long long *ticket)
+{
+    return submit_frames(c, in_fmt, planes, pitches, out_fmt, out_planes, out_pitches, dst_mask, mask_pitch, ticket,
+                         "sb_compositor_submit_frames");
 }
 
 int sb_compositor_wait(sb_compositor *c, unsigned long long ticket)

@@ -214,6 +214,24 @@ int warp_maps_upload(const Projector &p, const int rect[4], float *maps_dev, War
 int launch_repack_rgbx(const uint8_t *rgb, uint32_t *dst, long long pixels, cudaStream_t s);
 int launch_pack_rgbm(const uint8_t *rgb, long long rgb_pitch, const uint8_t *mask, long long mask_pitch, uint32_t *dst,
                      long long dst_pitch, int w, int h, cudaStream_t s);
+// true when launch_warp(jobs, n_jobs) serves job i with a kernel that reads WarpJob::src4 and never WarpJob::src
+bool warp_reads_src4_only(const WarpJob *jobs, int n_jobs, int i);
+// YUV 4:2:0 planes (sb_yuv.cu): NV12 has Y and the interleaved UV plane in `u` (v unused), I420 has Y, U and V.  Pitches
+// are in bytes and even.
+struct YuvPlanes {
+    const uint8_t *y, *u, *v;
+    long long ypitch, upitch, vpitch;
+};
+struct YuvOut {
+    uint8_t *y, *u, *v;
+    long long ypitch, upitch, vpitch;
+};
+// cv.cvtColor(COLOR_YUV2BGR_NV12 / _I420) of an even w x h frame into the packed 3-byte source (bgr != null) or the
+// word-per-pixel source of the warp kernel (bgrx != null, pitch in words)
+int launch_yuv420_to_src(int fmt, const YuvPlanes &in, int w, int h, uint8_t *bgr, long long bgr_pitch, uint32_t *bgrx,
+                         long long bgrx_pitch, cudaStream_t s);
+// cv.cvtColor(COLOR_BGR2YUV_I420) of an even w x h uint8 BGR image, chroma interleaved for NV12
+int launch_bgr_to_yuv420(int fmt, const uint8_t *bgr, long long bgr_pitch, int w, int h, const YuvOut &out, cudaStream_t s);
 // level `l` -> `l+1` of images [first, first+count)
 // `pyr` / `col`: the compact descriptors of level l for the same images (device pointers, `count` / `n` entries)
 // binary_masks: the caller guarantees that every mask byte of these images is 0 or 255 (used for l <= 2; sb_pyrdown_fast.cu)
@@ -266,6 +284,64 @@ static inline cudaError_t sb_copy2d(void *dst, size_t dpitch, const void *src, s
 {
     if (dpitch == width && spitch == width) return cudaMemcpyAsync(dst, src, width * height, kind, s);
     return cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, height, kind, s);
+}
+
+// YUV 4:2:0 frames (sb_pix_fmt): plane k's bytes per row and rows, and its offset / pitch in the dense layout -- cv2's
+// single (h * 3/2) x w array: Y, then UV (NV12) or U then V (I420), rows without padding
+inline int yuv_nplanes(int fmt) { return fmt == SB_PIX_NV12 ? 2 : 3; }
+inline size_t yuv_row_bytes(int fmt, int k, int w) { return k == 0 || fmt == SB_PIX_NV12 ? (size_t)w : (size_t)w / 2; }
+inline int yuv_rows(int k, int h) { return k == 0 ? h : h / 2; }
+inline size_t yuv_bytes(int w, int h) { return (size_t)w * h / 2 * 3; }
+inline size_t yuv_dense_offset(int fmt, int k, int w, int h)
+{
+    return k == 0 ? 0 : (size_t)w * h + (k == 2 ? yuv_row_bytes(fmt, 1, w) * (size_t)(h / 2) : 0);
+}
+// every plane the format uses is given, with a pitch that holds its row
+inline bool yuv_planes_ok(int fmt, const uint8_t *const planes[3], const size_t pitches[3], int w)
+{
+    if (!planes || !pitches) return false;
+    for (int k = 0; k < yuv_nplanes(fmt); ++k)
+        if (!planes[k] || pitches[k] < yuv_row_bytes(fmt, k, w)) return false;
+    return true;
+}
+inline YuvPlanes yuv_dense_planes(int fmt, const uint8_t *buf, int w, int h)
+{
+    YuvPlanes p;
+    p.y = buf;
+    p.ypitch = w;
+    p.u = buf + yuv_dense_offset(fmt, 1, w, h);
+    p.upitch = (long long)yuv_row_bytes(fmt, 1, w);
+    p.v = fmt == SB_PIX_NV12 ? nullptr : buf + yuv_dense_offset(fmt, 2, w, h);
+    p.vpitch = fmt == SB_PIX_NV12 ? 0 : (long long)yuv_row_bytes(fmt, 2, w);
+    return p;
+}
+inline YuvOut yuv_dense_out(int fmt, uint8_t *buf, int w, int h)
+{
+    const YuvPlanes p = yuv_dense_planes(fmt, buf, w, h);
+    return YuvOut{const_cast<uint8_t *>(p.y), const_cast<uint8_t *>(p.u), const_cast<uint8_t *>(p.v), p.ypitch, p.upitch, p.vpitch};
+}
+// the planes of a frame between host buffers and a dense device buffer `dev`: one copy per plane, or ONE copy when the host
+// planes lie densely in one buffer as well (the DMA engines reach PCIe line rate with long linear transfers)
+static inline cudaError_t yuv_copy(uint8_t *dev, const uint8_t *const host[3], const size_t pitches[3], int fmt, int w, int h,
+                                   cudaMemcpyKind kind, cudaStream_t s)
+{
+    const int np = yuv_nplanes(fmt);
+    bool dense = true;
+    for (int k = 0; k < np; ++k)
+        dense = dense && pitches[k] == yuv_row_bytes(fmt, k, w) && host[k] == host[0] + yuv_dense_offset(fmt, k, w, h);
+    if (dense) {
+        const bool up = kind == cudaMemcpyHostToDevice;
+        return cudaMemcpyAsync(up ? (void *)dev : (void *)host[0], up ? (const void *)host[0] : (const void *)dev, yuv_bytes(w, h), kind, s);
+    }
+    for (int k = 0; k < np; ++k) {
+        uint8_t *d = dev + yuv_dense_offset(fmt, k, w, h);
+        const size_t row = yuv_row_bytes(fmt, k, w);
+        const cudaError_t e = kind == cudaMemcpyHostToDevice
+                                  ? sb_copy2d(d, row, host[k], pitches[k], row, yuv_rows(k, h), kind, s)
+                                  : sb_copy2d((void *)host[k], pitches[k], d, row, row, yuv_rows(k, h), kind, s);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
 // Timelapser frame: src8 (uint8 x3, pitch in bytes) or src16 (int16 x3, pitch in ELEMENTS) pasted at (dx, dy) of a cw x ch canvas

@@ -439,6 +439,28 @@ int launch_repack_rgbx(const uint8_t *rgb, uint32_t *dst, long long pixels, cuda
     return launch_check("k_repack_rgbx");
 }
 
+// which fast warp kernel a batch of jobs qualifies for (launch_warp)
+static void classify_batch(const WarpJob *j, int cnt, bool &rgbm_only, bool &has_bm, bool &src4)
+{
+    rgbm_only = true, has_bm = false, src4 = true;
+    for (int i = 0; i < cnt; ++i) {
+        src4 = src4 && j[i].src4 != nullptr;
+        rgbm_only = rgbm_only && !j[i].xmap && j[i].dst_rgbm && !j[i].dst_rgb && !j[i].dst_mask && j[i].sw <= 32767 && j[i].sh <= 32767 &&
+                    j[i].sw >= 2 && j[i].sh >= 2 && j[i].rgbm_pitch % 2 == 0;
+        has_bm = has_bm || j[i].blend_mask || j[i].gain_mode;  // per-pixel extras anywhere in the batch
+    }
+}
+
+bool warp_reads_src4_only(const WarpJob *jobs, int n_jobs, int i)
+{
+    if (use_simple_kernels()) return false;
+    const int first = i - i % SB_WARP_BATCH;
+    const int cnt = n_jobs - first < SB_WARP_BATCH ? n_jobs - first : SB_WARP_BATCH;
+    bool rgbm_only, has_bm, src4;
+    classify_batch(jobs + first, cnt, rgbm_only, has_bm, src4);
+    return rgbm_only && src4;
+}
+
 int launch_warp(const WarpJob *jobs_host, int n_jobs, cudaStream_t s)
 {
     for (int first = 0; first < n_jobs; first += SB_WARP_BATCH) {
@@ -454,13 +476,8 @@ int launch_warp(const WarpJob *jobs_host, int n_jobs, cudaStream_t s)
         if (max_w <= 0 || max_h <= 0) continue;
         dim3 block(WARP_BX, WARP_BY), grid(div_up(max_w, WARP_BX), div_up(max_h, WARP_BY), cnt);
         if (!use_simple_kernels()) {
-            bool rgbm_only = true, has_bm = false, src4 = true;
-            for (int i = 0; i < cnt; ++i) {
-                src4 = src4 && B.j[i].src4 != nullptr;
-                rgbm_only = rgbm_only && !B.j[i].xmap && B.j[i].dst_rgbm && !B.j[i].dst_rgb && !B.j[i].dst_mask && B.j[i].sw <= 32767 && B.j[i].sh <= 32767 &&
-                            B.j[i].sw >= 2 && B.j[i].sh >= 2 && B.j[i].rgbm_pitch % 2 == 0;
-                has_bm = has_bm || B.j[i].blend_mask || B.j[i].gain_mode;  // per-pixel extras anywhere in the batch
-            }
+            bool rgbm_only, has_bm, src4;
+            classify_batch(B.j, cnt, rgbm_only, has_bm, src4);
             if (rgbm_only) {
                 dim3 grid2(div_up(max_w, 2 * WARP_BX), div_up(max_h, WARP_BY), cnt);
                 if (has_bm && src4)
